@@ -301,9 +301,22 @@ def issue_roofline(warp_inst_per_step, rows, steps_per_row, t_kernel, sm_mhz, n_
                        "scripts/probes/icache_probe.cu on this pool's B200 (profiles/r02_icache_probe.json)")
 
 
-def measure_config(ci, args, rank, world, local, steps, warmup, sampler=None, full=True, fp32_peak_tf=None):
+def dump_outputs(out_dir, arrays):
+    """One ``<name>.npy`` per output of the timed path (integers and float64 as float64, the rest as
+    float32), so that two builds can be compared output for output.  The largest config returns
+    well under 1 MB (Nsample+1 rewards, the knots, the bars), so nothing is sampled."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        a = v.detach().cpu().numpy() if hasattr(v, "detach") else np.asarray(v)
+        a = a.astype(np.float64 if a.dtype.kind in "iu" or a.dtype == np.float64 else np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure_config(ci, args, rank, world, local, steps, warmup, sampler=None, full=True, fp32_peak_tf=None,
+                   dump_dir=None):
     """Time config ci on this process group.  Returns the JSON fields of the config (rank 0: all
-    of them; other ranks: partial).  full=False skips the clocks / cpu arms (secondary blocks)."""
+    of them; other ranks: partial).  full=False skips the clocks / cpu arms (secondary blocks).
+    dump_dir: rank 0 writes there what the last timed step returned (dump_outputs)."""
     import torch
     import torch.distributed as dist
     from dial_mpc_b200 import random as drandom
@@ -337,7 +350,7 @@ def measure_config(ci, args, rank, world, local, steps, warmup, sampler=None, fu
         if use_graph:
             loop.step(cfg.Ndiffuse, env_step=2)
         else:
-            carry["rng"], carry["Y"], _ = mb.reverse_scan(state, carry["rng"], mb.shift(carry["Y"]), factors)
+            carry["rng"], carry["Y"], carry["info"] = mb.reverse_scan(state, carry["rng"], mb.shift(carry["Y"]), factors)
 
     def sync_all():
         torch.cuda.synchronize()
@@ -362,6 +375,13 @@ def measure_config(ci, args, rank, world, local, steps, warmup, sampler=None, fu
         evs.append((e0, e1))
     sync_all()
     t_wall = time.perf_counter() - t_wall0
+    if dump_dir is not None and rank == 0:
+        if use_graph:
+            outs = dict(Y=loop.Y, rng=loop.rng_host(), **loop.info())
+        else:
+            outs = dict(Y=carry["Y"], rng=carry["rng"],
+                        **{k: v for k, v in carry["info"].items() if k in ("rews", "qbar", "qdbar", "xbar")})
+        dump_outputs(dump_dir, outs)
     xwait = None
     if xst0 is not None:
         # device-measured time this rank's update kernels spent waiting for the slowest peer's flag
@@ -534,7 +554,8 @@ def run_own(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    head = measure_config(ci, args, rank, world, local, args.steps, args.warmup, sampler=sampler, fp32_peak_tf=fp32_peak)
+    head = measure_config(ci, args, rank, world, local, args.steps, args.warmup, sampler=sampler, fp32_peak_tf=fp32_peak,
+                          dump_dir=args.dump_outputs)
     others = {}
     if not args.only:
         todo = [i for i in (0, 1, 2, 3) if i != ci] if world == 1 else []
@@ -603,7 +624,11 @@ def main():
     ap.add_argument("--only", action="store_true", help="time only --config (no block for the other configs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--numpy-oracle", action="store_true", help="reference arm: NumPy oracle even if the C port is built")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of --config returned (knots Y, rng, rews, qbar, qdbar, xbar) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl own)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,5 +1,6 @@
 """TEST-ONLY python driver of the CPU warp emulator (tests/emul/libdial_emul.so)."""
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -20,7 +21,6 @@ def build(force=False, reward_source=None, defines=()):
             os.path.join(_DIR, "..", "..", "include", "dial_b200.h")]
     so, extra = _SO, []
     if reward_source is not None:
-        import hashlib
         reward_source = os.path.abspath(reward_source)
         tag = hashlib.sha256(open(reward_source, "rb").read()).hexdigest()[:12]
         so = os.path.join(_DIR, f"libdial_emul_custom_{tag}.so")
@@ -30,9 +30,17 @@ def build(force=False, reward_source=None, defines=()):
         so = so[:-3] + "_" + "_".join(d.replace("=", "-") for d in defines) + ".so"
         extra = extra + [f"-D{d}" for d in defines]
     if so not in _LIBS or force:
-        if force or not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
+        # content hash, not mtimes: a copied tree need not keep them, and a built tree may be read-only
+        h = hashlib.sha256()
+        for s in srcs:
+            h.update(open(s, "rb").read())
+        h.update(" ".join(f"-D{d}" for d in defines).encode())
+        digest, side = h.hexdigest(), so + ".sha256"
+        if force or not (os.path.exists(so) and os.path.exists(side) and open(side).read().strip() == digest):
             subprocess.check_call(["g++", "-O1", "-std=c++17", "-I", _DIR, "-shared", "-fPIC"] + extra +
                                   ["-o", so, os.path.join(_DIR, "emul_main.cpp")])
+            with open(side, "w") as f:
+                f.write(digest)
         _LIBS[so] = C.CDLL(so)
     return _LIBS[so]
 

@@ -49,10 +49,13 @@ def test_two_rank_sharding_matches_single_rank():
     Ybar = (rng.standard_normal((4, 12)) * 0.3).astype(np.float32)
     single = {}
     _run(0, 1, _free_port(), eps, Ybar, single)
-    mgr = mp.Manager()
-    ret = mgr.dict()
-    mp.spawn(_run, args=(2, _free_port(), eps, Ybar, ret), nprocs=2, join=True)
-    r0, r1, s0 = ret[0], ret[1], single[0]
+    # a spawned manager: forking this (multi-threaded) process leaves its OpenBLAS thread pool hung, and the
+    # next threaded np.linalg call of a later test never returns
+    with mp.get_context("spawn").Manager() as mgr:
+        ret = mgr.dict()
+        mp.spawn(_run, args=(2, _free_port(), eps, Ybar, ret), nprocs=2, join=True)
+        r0, r1 = ret[0], ret[1]
+    s0 = single[0]
     # per-sample rewards do not depend on the shard: bitwise identical
     assert np.array_equal(r0["rews"], s0["rews"]) and np.array_equal(r1["rews"], s0["rews"])
     # every rank holds the same control update; bars agree with the single-rank run
